@@ -3,6 +3,11 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's sm_100a path
     python bench.py --impl reference --gpus N --steps K ...   # the reference arithmetic on the box's host cores
+    python bench.py ... --dump-outputs DIR                    # + what the last timed step returned, as DIR/*.npy
+
+--steps K is the number of timed steps of each GPU-timed loop (device-resident, end to end, eager peer). The inputs
+(seeded weights, synthetic batches, host random stream) are the same on every run with the same arguments, so the
+dumped outputs of two builds can be compared array for array.
 
 Workload (BASELINE.json configs[1]): FLUX-VAE config ch=128, ch_mult=1,2,4,4, z=16, 256x256 synthetic images,
 one step = Encoder -> clamp -> reg -> Decoder -> GradNorm -> LPIPS(eval) + 0.1*mean(z^2) (+ pooled L1 at the reference's
@@ -252,6 +257,45 @@ def profile_conv_kernels(tr, batch_dev):
     return out
 
 
+DUMP_BYTES = 64_000_000
+
+
+def host_outputs(out, prefix=""):
+    """What Trainer.step returned, flattened to {name: float32/float64 numpy array} on the host (nested dicts become
+    `outer.inner`). Copy before the next step: a CUDA-graph replay reuses the same output buffers."""
+    import numpy as np
+
+    arrs = {}
+    for k, v in out.items():
+        name = prefix + k
+        if isinstance(v, dict):
+            arrs.update(host_outputs(v, name + "."))
+        elif torch.is_tensor(v):
+            v = v.detach()
+            arrs[name] = v.cpu().numpy() if v.dtype == torch.float64 else v.float().cpu().numpy()
+        else:
+            arrs[name] = np.asarray(v, dtype=np.float64)
+    return arrs
+
+
+def dump_outputs(arrs, outdir):
+    """Writes each array as outdir/<name>.npy, DUMP_BYTES in all (1 KiB per file kept for the .npy header). Smallest
+    arrays first, each gets an equal share of what is left; an array larger than its share is replaced by a fixed sample
+    of its flattened elements (seed 0, sorted positions), so two runs with the same arguments write comparable files."""
+    import numpy as np
+
+    os.makedirs(outdir, exist_ok=True)
+    left = DUMP_BYTES - 1024 * len(arrs)
+    for i, (name, a) in enumerate(sorted(arrs.items(), key=lambda kv: kv[1].nbytes)):
+        keep = max(1, left // (len(arrs) - i) // a.itemsize)
+        if a.size > keep:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, keep, replace=False))
+            sys.stderr.write(f"dump-outputs: {name} {a.shape}: fixed sample of {keep} of {a.size} elements\n")
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(outdir, name + ".npy"), a)
+        left -= a.nbytes
+
+
 _JSON_OUT = None
 
 
@@ -355,7 +399,7 @@ def eager_b200_leg(cfg, B, world, rank, device, steps, warmup):
             for i in range(max(2, min(warmup, 3))):
                 step(batches[i % 2])
             torch.cuda.synchronize()
-            k = max(2, min(steps, 5))
+            k = steps
             if world > 1:
                 dist.barrier()
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -427,7 +471,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-eager", action="store_true", help="skip the PyTorch-eager-on-B200 peer leg")
     ap.add_argument("--no-graph", action="store_true", help="run the step eagerly instead of as one CUDA-graph replay")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned as DIR/<name>.npy (rank 0, 64 MB at most)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.gan and args.config == "lpips":
         args.config = "gan"
     cfg = CONFIGS[args.config]
@@ -492,6 +540,7 @@ def main():
     barrier()
     ms = e0.elapsed_time(e1) / K
     launches = (native.launch_count() - l0)
+    dumped = host_outputs(out) if args.dump_outputs and rank == 0 else None
     graphed = tr.graph_launches_per_step is not None
     if graphed:  # replays do not pass through the C entry points: kernels per replay (counted at capture) x replays
         launches = tr.graph_launches_per_step * K
@@ -594,6 +643,8 @@ def main():
                                               f"of the reference arithmetic, torch CPU fp32, {threads} threads); the "
                                               "reference tree is unpackaged Python and cannot be installed/travel"}
         emit_json(line)
+        if dumped is not None:
+            dump_outputs(dumped, args.dump_outputs)
     # release the captured step (its graph holds NCCL work) before tearing the process group down: with a live graph
     # destroy_process_group() hung until the launcher's timeout (N=2, round 2)
     tr = None

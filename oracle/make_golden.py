@@ -261,6 +261,24 @@ def ckpt_case(name="ref_ckpt_step_small"):
     print("wrote", path, os.path.getsize(path), "bytes,", len(ddp.state_dict()), "tensors")
 
 
+def init_case(name="ref_init_seed123"):
+    """The reference's initial weights after torch.manual_seed(123) (vae_trainer.py:374-378) for a VAE with two res
+    blocks per level and the HR decoder level: parameter creation order and init calls decide every value. 2.3M floats
+    do not fit a fixture, so each tensor is stored as shape + SHA-256 of its float32 bytes (bit-exact either way)."""
+    import hashlib
+    import json
+
+    torch.manual_seed(123)
+    m = ref_ae.VAE(64, 3, 32, 3, [1, 2], 2, 4, False, True, False)
+    table = [{"key": k, "shape": list(v.shape), "dtype": str(v.dtype).replace("torch.", ""),
+              "sha256": hashlib.sha256(v.detach().contiguous().numpy().tobytes()).hexdigest()}
+             for k, v in m.state_dict().items()]
+    path = os.path.join(OUT, name + ".json")
+    with open(path, "w") as f:
+        f.write("[\n" + ",\n".join(json.dumps(e) for e in table) + "\n]\n")
+    print("wrote", path, len(table), "tensors")
+
+
 def _sub(tag, grads, res, keys, budget=60_000):
     """Full gradient tensors are too large for a fixture at ch=128: store every s-th element of the flattened tensor
     (s = smallest stride keeping <= budget elements; s == 1 keeps it whole) as `<tag>grad::<key>` and s as
@@ -392,7 +410,7 @@ if __name__ == "__main__":
     only = sys.argv[1:]
     if only:  # e.g. `python oracle/make_golden.py flux_step flux_hr` (the ch=128 cases take minutes of CPU time)
         for c in only:
-            {"flux_step": flux_step_case, "flux_hr": flux_hr_case, "ckpt": ckpt_case}[c]()
+            {"flux_step": flux_step_case, "flux_hr": flux_hr_case, "ckpt": ckpt_case, "init": init_case}[c]()
         dist.destroy_process_group()
         sys.exit(0)
     vae_case("vae_small", VO.VAEConfig(resolution=32, ch=32, ch_mult=(1, 2), num_res_blocks=2, z_channels=4), 2, 32)
@@ -407,5 +425,6 @@ if __name__ == "__main__":
     flux_step_case()
     flux_hr_case()
     ckpt_case()
+    init_case()
     dist.destroy_process_group()
     print("all golden fixtures written to", OUT)
